@@ -4,9 +4,11 @@
 GPS L1 C/A, 32 channels, 25 Msps synthetic IQ, 3 taps (E/P/L), 1 s of signal per step
 (1000 epochs of 25000 samples per channel => 8e8 channel-samples per step).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
-One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
+One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.  --dump-outputs DIR writes the taps
+the last timed step returned to DIR/trk_taps.npy, so that two builds can be compared output for output (the inputs
+are generated from fixed seeds).
 """
 from __future__ import annotations
 
@@ -21,6 +23,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree: no __pycache__ beside the sources
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -760,7 +763,11 @@ def main():
     ap.add_argument("--no-acq", action="store_true")
     ap.add_argument("--no-loop", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the sustained leg, the other BASELINE configs and the coalescer leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the taps of the last timed step (float32 [items, taps, re/im], items epoch-major) to DIR/trk_taps.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
@@ -833,6 +840,9 @@ def main():
         ev[k + 1].record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "trk_taps.npy"), out_dev.cpu().numpy())
     total_ms = ev[0].elapsed_time(ev[-1])
     launches = eng.launch_count() - l0
     # cross-check with the library's own CUDA-event timer on the engine stream (one extra step)

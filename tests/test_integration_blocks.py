@@ -10,6 +10,7 @@ This is BASELINE.json configs[0] ("GPS L1 C/A, 1 channel, 4 Msps file source, pc
 run through general_work on both sides.  CPU-only tests cover the oracle chain itself, the build / link / symbol check
 of the B200 sources and the factory patch; `-m gpu` tests are the parity tests.
 """
+import hashlib
 import os
 import shutil
 import subprocess
@@ -21,6 +22,9 @@ import blocks_itf as bi
 from gnss_synth import make_iq
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# the reference chain's results on gps_signal (and the code table it is made from), written by tests/golden/make_golden.py
+# from oracle/_ref/liboracle_ref_blocks.so: the CPU tests of the oracle chain read them from here
+GOLDEN = os.path.join(ROOT, "tests", "golden", "blocks_ref_golden.npz")
 FS = 4_000_000
 E1C_SECONDARY = "0011100000001010110110010"  # GALILEO_E1_C_SECONDARY_CODE, src/core/system_parameters/Galileo_E1.h
 
@@ -52,15 +56,44 @@ def b200lib():
 
 
 @pytest.fixture(scope="module")
-def gps_signal(reflib):
+def gold():
+    return np.load(GOLDEN)
+
+
+def make_gps_signal(code):
     """2.6 s of GPS L1 C/A PRN 1 at 4 Msps: Doppler 1680 Hz, code delay 524 samples (the parameters of the reference's
     GPS_L1_CA_ID_1_Fs_4Msps_2ms.dat known answer, gps_l1_ca_pcps_acquisition_test.cc:302-303), 20 ms navigation bits."""
     rng = np.random.default_rng(7)
     bits = rng.choice([-1.0, 1.0], 400)
-    code = bi.code_table(reflib, "G", "1C", 1)
     sv = dict(prn=1, doppler=1680.0, code_phase_chips=(-524 * 1.023e6 / FS) % 1023, cn0=49.0, symbols=bits, periods_per_symbol=20)
     iq = make_iq({1: code}, FS, int(FS * 2.6), [sv], seed=1)
     return iq, bits
+
+
+@pytest.fixture(scope="module")
+def gps_signal(gold):
+    """make_gps_signal over the reference generator's PRN 1 replica (stored)."""
+    return make_gps_signal(gold["code/G/1C/1"])
+
+
+def stored_chain(gold, name, iq):
+    """run_chain's result for the reference blocks, as stored for the samples `iq` (checked by digest)."""
+    assert hashlib.sha256(np.ascontiguousarray(iq).tobytes()).digest() == gold[f"{name}/iq_sha"].tobytes(), \
+        "the stored reference run was made on other samples: regenerate tests/golden/blocks_ref_golden.npz"
+    acq = gold[f"{name}/acq"]
+    return dict(acq=(float(acq[0]), float(acq[1]), int(acq[2])), acq_events=gold[f"{name}/acq_events"].tolist(),
+                started=int(gold[f"{name}/started"]), out=gold[f"{name}/out"].view(bi.SYNCHRO_DTYPE),
+                trk_events=gold[f"{name}/trk_events"].tolist())
+
+
+# the reference chain runs of the CPU tests below: name -> (conf overrides, arch, seconds of gps_signal)
+REF_RUNS = {
+    "c1": (dict(), "simd", 2.6),
+    "states_3_4": ({"Tracking_1C.extend_correlation_symbols": 20, "Tracking_1C.pll_bw_narrow_hz": 5.0, "Tracking_1C.dll_bw_narrow_hz": 0.75,
+                    "Tracking_1C.early_late_space_narrow_chips": 0.15, "Tracking_1C.pll_filter_order": 2}, "simd", 2.6),
+    "generic_1s8": (dict(), "generic", 1.8),
+    "simd_1s8": (dict(), "simd", 1.8),
+}
 
 
 def run_chain(lib, conf, acq_impl, trk_impl, iq, prn=1, system="G", signal="1C", acq_role="Acquisition_1C", trk_role="Tracking_1C"):
@@ -79,12 +112,12 @@ def run_chain(lib, conf, acq_impl, trk_impl, iq, prn=1, system="G", signal="1C",
 
 
 # ---------------------------------------------------------------------------------------------- CPU: oracle chain
-def test_reference_chain_c1_known_answer(reflib, gps_signal):
+def test_reference_chain_c1_known_answer(gold, gps_signal):
     """The reference's own acquisition + FSM + tracking blocks on the C1-shaped signal: delay 524 samples, Doppler in
     the 1750 Hz bin, FSM goes to tracking without an "events" message, tracking converges to 1680 Hz, finds the bit
     edges and delivers the transmitted navigation bits (up to the Costas sign)."""
     iq, bits = gps_signal
-    r = run_chain(reflib, base_conf(), "GPS_L1_CA_PCPS_Acquisition", "GPS_L1_CA_DLL_PLL_Tracking", iq)
+    r = stored_chain(gold, "c1", iq)
     assert r["acq"] == (524.0, 1750.0, 4000)
     assert r["started"] == 1 and r["acq_events"] == []  # positive acquisition went straight to the FSM (pcps_acquisition.cc:322-326)
     out = r["out"]
@@ -106,29 +139,25 @@ def test_reference_chain_c1_known_answer(reflib, gps_signal):
     assert abs(np.sum(got * want)) == len(got)
 
 
-def test_reference_chain_extended_integration_states_3_4(reflib, gps_signal):
+def test_reference_chain_extended_integration_states_3_4(gold, gps_signal):
     """extend_correlation_symbols = 20: after bit synchronisation the reference block alternates states 3/4, switches
     to the narrow correlator spacing in place and keeps delivering one symbol per 20 ms."""
     iq, _ = gps_signal
     # (pll_filter_order 2: with the default 3rd-order filter and a 5 Hz narrow bandwidth the reference's own loop walks off
-    #  after the switch on this signal - as found, not a property under test)
-    conf = base_conf(**{"Tracking_1C.extend_correlation_symbols": 20, "Tracking_1C.pll_bw_narrow_hz": 5.0, "Tracking_1C.dll_bw_narrow_hz": 0.75,
-                        "Tracking_1C.early_late_space_narrow_chips": 0.15, "Tracking_1C.pll_filter_order": 2})
-    r = run_chain(reflib, conf, "GPS_L1_CA_PCPS_Acquisition", "GPS_L1_CA_DLL_PLL_Tracking", iq)
+    #  after the switch on this signal - as found, not a property under test; REF_RUNS["states_3_4"] holds the conf)
+    r = stored_chain(gold, "states_3_4", iq)
     out = r["out"]
     assert len(out) >= 50 and r["trk_events"] == []
     assert abs(np.mean(out["Carrier_Doppler_hz"][-20:]) - 1680.0) < 1.0
     assert np.all(np.abs(np.diff(out["Tracking_sample_counter"].astype(np.int64)) - 80000) <= 2)
 
 
-def test_reference_generic_vs_simd_drift(reflib, gps_signal):
+def test_reference_generic_vs_simd_drift(gold, gps_signal):
     """Calibration of the parity bounds used below: the reference chain with its generic kernels against itself with its
     SIMD kernels (same blocks, same samples).  Closed-loop tracking amplifies 1e-6 correlator differences."""
     iq, _ = gps_signal
-    reflib.itf_select_arch(b"generic")
-    a = run_chain(reflib, base_conf(), "GPS_L1_CA_PCPS_Acquisition", "GPS_L1_CA_DLL_PLL_Tracking", iq[:int(FS * 1.8)])
-    reflib.itf_select_arch(b"simd")
-    b = run_chain(reflib, base_conf(), "GPS_L1_CA_PCPS_Acquisition", "GPS_L1_CA_DLL_PLL_Tracking", iq[:int(FS * 1.8)])
+    a = stored_chain(gold, "generic_1s8", iq[:int(FS * 1.8)])
+    b = stored_chain(gold, "simd_1s8", iq[:int(FS * 1.8)])
     assert a["acq"] == b["acq"]
     n = min(len(a["out"]), len(b["out"]))
     assert n >= 20 and abs(len(a["out"]) - len(b["out"])) <= 1

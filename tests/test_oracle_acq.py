@@ -1,6 +1,7 @@
 """Pins for the acquisition oracle (oracle/port_acq.c, oracle/acq_np.py).
 
-* sincos / index_max C ports are checked BIT-EXACT against the reference's own kernels.
+* sincos / index_max C ports are checked BIT-EXACT against the reference's own kernels (their outputs stored in
+  tests/golden/ref_calls.npz, see tests/ref_golden.py).
 * The numpy grid search is checked against the reference's own generator-based known answer
   (tests/unit-tests/signal-processing-blocks/acquisition/gps_l1_ca_pcps_acquisition_gsoc2013_test.cc:
   207-263: fs 4 Msps, PRN 10 (we use the same numbers), Doppler 750 Hz, delay 600 chips,
@@ -15,10 +16,7 @@ import numpy as np
 import pytest
 
 from gnss_synth import make_iq
-
-
-def _bits(a):
-    return np.ascontiguousarray(a).view(np.uint32)
+from ref_golden import same_bits
 
 
 @pytest.mark.parametrize("n", [4000, 25000, 8111, 13])
@@ -31,7 +29,7 @@ def test_sincos_ports_bitexact(oracle, ref, n, freq):
         got = np.empty(n, np.complex64)
         ph = C.c_float(0.0)
         fn(C.c_void_p(got.ctypes.data), C.c_float(float(inc)), C.byref(ph), C.c_uint(n))
-        assert np.array_equal(_bits(got), _bits(want)), variant
+        assert same_bits(got, want), variant
         assert np.float32(ph.value) == np.float32(ph_w)
 
 

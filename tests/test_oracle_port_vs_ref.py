@@ -5,14 +5,12 @@ Shapes follow the reference QA: vlen 8111, puppet parameters
  L=2046, step=(L+0.1)/N, rem=-0.234, shifts {-0.1,0,0.1};
  ..._32fc_32f_rotator_dotprodxnpuppet_32fc.h:31-55: rem 0.25 rad, step 0.1 rad, 3 taps)
 plus the BASELINE shapes (N=25000 L=1023 3 taps; N=200000 L=8184 5 taps) and ragged sizes.
+The reference's outputs for these calls are stored in tests/golden/ref_calls.npz (tests/ref_golden.py).
 """
 import numpy as np
 import pytest
 
-
-def _bits(a):
-    a = np.ascontiguousarray(a)
-    return a.view(np.uint32 if a.dtype.itemsize == 4 else np.uint64)
+from ref_golden import same_bits
 
 
 CASES = [
@@ -34,7 +32,7 @@ def test_resampler_generic_bitexact(oracle, ref, n, L, shifts, rem, step):
     code = rng.choice([-1.0, 1.0], L).astype(np.float32)
     a = oracle.port.resampler(0, code, rem, step, shifts, n)
     b = ref.resampler("generic", code, rem, step, shifts, n)
-    assert np.array_equal(_bits(a), _bits(b))
+    assert same_bits(a, b)
 
 
 @pytest.mark.parametrize("n,L,shifts,rem,step", CASES)
@@ -45,7 +43,7 @@ def test_resampler_avx_bitexact(oracle, ref, variant, n, L, shifts, rem, step):
     code = rng.standard_normal(L).astype(np.float32)
     a = oracle.port.resampler(1, code, rem, step, shifts, n)
     b = ref.resampler(variant, code, rem, step, shifts, n)
-    assert np.array_equal(_bits(a), _bits(b))
+    assert same_bits(a, b)
 
 
 @pytest.mark.parametrize("n,taps", [(8111, 3), (25000, 3), (200000, 5), (4096, 1), (100, 3), (15, 2), (16, 2), (1041, 4)])
@@ -57,8 +55,8 @@ def test_rotator_generic_bitexact(oracle, ref, n, taps):
     ph0 = np.complex64(np.cos(0.25) - 1j * np.sin(0.25))
     a, pa = oracle.port.rotator_generic(iq, inc, ph0, codes)
     b, pb = ref.rotator("generic", iq, inc, ph0, codes)
-    assert np.array_equal(_bits(a), _bits(b))
-    assert np.array_equal(_bits(np.array([pa])), _bits(np.array([pb])))
+    assert same_bits(a, b)
+    assert same_bits(np.array([pa]), np.array([pb]))
 
 
 @pytest.mark.parametrize("n,taps", [(8111, 3), (25000, 3), (200000, 5), (4096, 1), (100, 3), (15, 2), (16, 2), (1041, 4)])
@@ -71,8 +69,8 @@ def test_rotator_avx_bitexact(oracle, ref, variant, n, taps):
     ph0 = np.complex64(np.cos(0.4) - 1j * np.sin(0.4))
     a, pa = oracle.port.rotator_avx(iq, inc, ph0, codes)
     b, pb = ref.rotator(variant, iq, inc, ph0, codes)
-    assert np.array_equal(_bits(a), _bits(b))
-    assert np.array_equal(_bits(np.array([pa])), _bits(np.array([pb])))
+    assert same_bits(a, b)
+    assert same_bits(np.array([pa]), np.array([pb]))
 
 
 def test_rotator_avx_vs_generic_within_reference_tolerance(ref):
@@ -105,7 +103,7 @@ def test_multicorrelator_class_bitexact(oracle, ref, arch, refarch, n, L, shifts
     ref.mc_destroy(h)
     ref.select_arch("a_avx")
     a = oracle.port.multicorrelator(arch, iq, code, shifts, rem_carr, dphi, rem_code, step)
-    assert np.array_equal(_bits(a), _bits(b))
+    assert same_bits(a, b)
 
 
 def test_hd_resampler_bitexact(oracle, ref):
@@ -115,7 +113,7 @@ def test_hd_resampler_bitexact(oracle, ref):
         code = rng.standard_normal(L).astype(np.float32)
         a = oracle.port.hd_resampler(code, -0.234, step, 1e-9, shifts, n)
         b = ref.hd_resampler("generic", code, -0.234, step, 1e-9, shifts, n)
-        assert np.array_equal(_bits(a), _bits(b))
+        assert same_bits(a, b)
 
 
 @pytest.mark.parametrize("variant", ["a_avx", "u_avx"])
@@ -129,7 +127,7 @@ def test_hd_resampler_avx_bitexact(oracle, ref, variant):
         code = rng.standard_normal(L).astype(np.float32)
         a = oracle.port.hd_resampler_avx(code, 0.37, step, rate, shifts, n)
         b = ref.hd_resampler(variant, code, 0.37, step, rate, shifts, n)
-        assert np.array_equal(_bits(a), _bits(b)), (variant, n)
+        assert same_bits(a, b), (variant, n)
 
 
 def test_hd_rotator_bitexact(oracle, ref):
@@ -142,8 +140,8 @@ def test_hd_rotator_bitexact(oracle, ref):
     ph0 = np.complex64(np.cos(0.4) - 1j * np.sin(0.4))
     a, pa = oracle.port.hd_rotator_generic(iq, inc, rate, ph0, codes)
     b, pb = ref.hd_rotator("generic", iq, inc, rate, ph0, codes)
-    assert np.array_equal(_bits(a), _bits(b))
-    assert np.array_equal(_bits(np.array([pa])), _bits(np.array([pb])))
+    assert same_bits(a, b)
+    assert same_bits(np.array([pa]), np.array([pb]))
 
 
 def test_f64_truth_bounds_float_paths(oracle):
